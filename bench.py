@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          (N > 1: launched by torch.distributed.run)
   python bench.py --impl reference ...                   the reference's own CPU implementation
+  python bench.py ... --dump-outputs DIR                 also save the last timed step's output (DIR/output.npy)
 
 Workload (BASELINE.json configs[1]): batch 1024 stereo streams per GPU, 48 kHz presetDefault,
 0.8x time-stretch (outputSamples = 0.8 * inputSamples, cmd/main.cpp:27,37 semantics), synthetic
@@ -79,6 +80,21 @@ def synth_input(batch, n, seed0=0):
     rng = np.random.default_rng(1234 + seed0)
     x += 0.01 * rng.standard_normal(x.shape)
     return x.astype(np.float32)
+
+
+DUMP_STREAMS = 64
+
+
+def dump_outputs(out_dir, y_dev):
+    """DIR/output.npy: what the last timed process() call returned, float32 [streams][channels][samples], for a fixed
+    seeded sample of DUMP_STREAMS streams of the batch in ascending order (the whole batch when it is smaller), so that
+    two builds run with the same arguments can be compared output for output."""
+    import torch
+
+    streams = np.sort(np.random.default_rng(0).choice(y_dev.shape[0], min(DUMP_STREAMS, y_dev.shape[0]), replace=False))
+    y = y_dev[torch.from_numpy(streams).to(y_dev.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output.npy"), y)
 
 
 # ------------------------------------------------------------------------------------ clocks
@@ -496,7 +512,13 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true", help="skip the child runs of BASELINE configs[2] / [3]")
     ap.add_argument("--sweep-filter", default="", help="config 5: only the points whose 'preset:num/den' contains this string (e.g. presetDefault:5/4)")
     ap.add_argument("--live", action="store_true", help="the live / streaming caller (seek + process(0, 128) per quantum), batch 1024 stereo")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's output of the device-resident path to DIR/output.npy (float32, %d sampled streams)" % DUMP_STREAMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.live or args.config == 5 or args.impl == "reference"):
+        ap.error("--dump-outputs applies to the device-resident path of --config 2, 3 or 4")
     if args.pcm16_probe:
         pcm16_probe(args)
         return
@@ -578,6 +600,8 @@ def main():
     clk = clocks.stop()
     total, tmax = reduce_throughput(w["samples_per_step"] * args.steps, ms / 1e3, dist if world > 1 else None, dev)
     value = total / tmax
+    if args.dump_outputs and rank == 0:  # y_dev still holds the last timed step; later passes overwrite it
+        dump_outputs(args.dump_outputs, y_dev)
 
     if args.no_e2e:
         if rank == 0:
@@ -685,7 +709,7 @@ def main():
         other_configs = {}
         for c in (3, 4):
             try:
-                r = subprocess.run([sys.executable, os.path.abspath(__file__), "--config", str(c), "--steps", "5", "--no-e2e"],
+                r = subprocess.run([sys.executable, os.path.abspath(__file__), "--config", str(c), "--steps", str(args.steps), "--no-e2e"],
                                    capture_output=True, text=True, timeout=240)
                 other_configs["config%d" % c] = json.loads(r.stdout.strip().splitlines()[-1]) if r.returncode == 0 else {"unavailable": (r.stderr or "failed")[-200:]}
             except Exception as ex:  # noqa: BLE001

@@ -31,9 +31,9 @@ def _segment():
 
 
 class LiveBatch:
-    def __init__(self, engine, sample_rate, bank=None, capacity=0):
+    def __init__(self, engine, sample_rate, bank="auto", capacity=0):
         """bank: "torch" (CUDA tensor), "numpy" (the emulated library's "device" memory is host memory) or None for host
-        mode; default: "torch" when the engine has b200s_live_seek and a GPU is there, else host mode."""
+        mode; "auto" (default): "torch" when the engine has b200s_live_seek and a GPU is there, else host mode."""
         self.eng, self.sr = engine, float(sample_rate)
         self.S, self.C = engine.batch, engine.channels()
         self.buffer_length = engine.inputLatency() + engine.outputLatency()  # :205-207
@@ -41,13 +41,15 @@ class LiveBatch:
         self.out_lat_s = engine.outputLatency() / self.sr
         self.time_maps = [[_segment()] for _ in range(self.S)]
         self.current_sample = 0  # currentTime * sampleRate of the audio context
-        if bank is None and hasattr(engine, "live_seek"):
-            try:
-                import torch
+        if bank == "auto":
+            bank = None
+            if hasattr(engine, "live_seek"):
+                try:
+                    import torch
 
-                bank = "torch" if torch.cuda.is_available() else None
-            except ImportError:
-                bank = None
+                    bank = "torch" if torch.cuda.is_available() else None
+                except ImportError:
+                    pass
         self.bank_kind = bank
         self.audio_start = np.zeros(self.S, np.int64)  # sample index of the first stored sample (audioBuffersStart)
         self.audio_len = np.zeros(self.S, np.int64)

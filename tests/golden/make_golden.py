@@ -9,7 +9,11 @@
 
 Each fixture: the first 16 blocks (+ latency) of output for one stream of a BASELINE config,
 driven with 480-sample output chunks, plus the input and the KATs of SURVEY.md section 8(c).
-The GPU box has no /root/reference, so these small files are what travels.
+Outputs too long to store whole are kept as a SHA-256 digest (bit-exact checks) or as an evenly
+spaced sample (statistical checks): see `header_cases` and `bench_shape`.  The tests need only
+these files, never the reference itself.
+
+  python tests/golden/make_golden.py [configs] [header_cases] [bench_shape]   (default: all)
 """
 import os
 import sys
@@ -25,7 +29,49 @@ from oracle.hdrref import CpuStretch  # noqa: E402
 from oracle.wasmref import WasmStretch  # noqa: E402
 
 
+def record(out, key, y, n_sample=512):
+    out[key + "_shape"] = np.array(y.shape)
+    out[key + "_sha256"] = signals.digest(y)
+    out[key + "_sample"] = y.reshape(-1)[signals.sample_positions(y.size, n_sample)]
+
+
+def header_cases():
+    """tests/test_oracle_pinning.py: the header on signals.HEADER_CASES and on the API sequence."""
+    out = {}
+    x = signals.header_case_input()
+    for i, (cfg, ratio, chunk) in enumerate(signals.HEADER_CASES):
+        h = CpuStretch("hdr")
+        cfg(h)
+        record(out, "case%d" % i, signals.run_single(h, x, ratio, chunk))
+    record(out, "api_sequence", signals.header_api_sequence(CpuStretch("hdr")))
+    np.savez_compressed(os.path.join(HERE, "reference_header_cases.npz"), **out)
+
+
+def bench_shape():
+    """tests/test_gpu_parity.py::test_benchmark_shape_vs_oracle: the shipped binary on stream 0 of config 2 at the
+    benchmark's shape (three calls of 32 blocks), 4096 evenly spaced positions per channel."""
+    cfg, C, sr, ratio, _ = signals.CONFIGS["config2_stereo_0p8x"]
+    n_out = 32 * int(sr * 0.03)
+    n_in = int(round(n_out / ratio))
+    x = np.stack([signals.harmonic(3 * n_in, sr, 0, c) for c in range(C)])
+    w = WasmStretch()
+    cfg(w)
+    y = signals.run_single(w, x, ratio, n_out)
+    idx = signals.sample_positions(y.shape[-1], 4096)
+    np.savez_compressed(os.path.join(HERE, "config2_bench_shape_wasm.npz"), x_sha256=signals.digest(x), wasm=y[:, idx])
+
+
 def main():
+    what = sys.argv[1:] or ["configs", "header_cases", "bench_shape"]
+    if "header_cases" in what:
+        header_cases()
+    if "bench_shape" in what:
+        bench_shape()
+    if "configs" in what:
+        configs()
+
+
+def configs():
     for name, (cfg, C, sr, ratio, kind) in signals.CONFIGS.items():
         H = int(sr * 0.03) if "cheaper" not in name else int(sr * 0.04)
         n_out = 16 * H + 2 * int(sr * 0.12)

@@ -1,4 +1,6 @@
 """Deterministic synthetic audio used by tests, golden vectors and bench.py (SURVEY.md section 8(d))."""
+import hashlib
+
 import numpy as np
 
 
@@ -56,6 +58,18 @@ def run_batch(obj, x, ratio_out, chunk_out):
     return np.concatenate(outs, axis=-1)
 
 
+# ---- compact golden records of long outputs: an exact digest plus an evenly spaced sample for diagnostics
+def digest(y):
+    """SHA-256 of float32 samples; -0.0 counts as 0.0, so equal digests mean np.array_equal."""
+    y = np.ascontiguousarray(np.asarray(y, np.float32) + np.float32(0), "<f4")
+    return np.frombuffer(hashlib.sha256(y.tobytes()).digest(), np.uint8)
+
+
+def sample_positions(n, k):
+    """k evenly spaced positions in [0, n)."""
+    return np.unique(np.linspace(0, n - 1, min(n, k)).round().astype(np.int64))
+
+
 # piecewise-linear frequency maps (setFreqMap with a tabulated function; frequencies as multiples of the sample rate)
 PWL_MONOTONE = (np.array([0.0, 0.02, 0.08, 0.2, 0.5], np.float32), np.array([0.0, 0.03, 0.1, 0.21, 0.5], np.float32))
 # not monotone: the band between 0.06 and 0.1 folds back below what the band under it maps to, so consecutive peaks can
@@ -102,3 +116,42 @@ CONFIGS = {
     "config4_formant": (cfg_config4, 2, 48000, 1.0, "harmonic"),
     "config5_cheaper_2x": (cfg_cheaper, 1, 48000, 2.0, "harmonic"),
 }
+
+
+# the oracle against the unmodified reference header, beyond the golden configurations: (configure fn, out/in ratio,
+# output chunk), all on header_case_input()
+HEADER_CASES = [
+    (lambda o: (o.presetDefault(2, 48000.0), o.setTransposeSemitones(-5, 0)), 1.5, 4800),
+    (lambda o: (o.presetCheaper(2, 48000.0, False), o.setTransposeSemitones(4, 0.2), o.setFormantSemitones(3, False), o.setFormantBase(0)), 1.0, 480),
+    (lambda o: (o.configure(2, 1000, 250, True), o.setFreqMapQuadratic(1.2, 0.5)), 0.9, 333),
+    (lambda o: o.presetDefault(2, 44100.0), 2.5, 441),  # > 2x: exercises the RNG path of the header
+    # setFreqMap with a piecewise-linear function: monotone, and one that folds back (non-monotone output map)
+    (lambda o: (o.configure(2, 1000, 250, False), o.setFreqMapTable(*PWL_MONOTONE)), 1.0, 500),
+    (lambda o: (o.presetDefault(2, 48000.0), o.setFreqMapTable(*PWL_FOLDING)), 1.25, 2880),
+]
+
+
+def header_case_input():
+    return np.stack([harmonic(30000, 48000, 1, 0), harmonic(30000, 48000, 1, 1)])
+
+
+def header_api_sequence(o):
+    """seek / silence bypass / flush / reset / outputSeek / exact on a one-stream CPU object, outputs concatenated."""
+    x = harmonic(60000, 48000)[None]
+    o.presetDefault(1, 48000.0)
+    o.setTransposeSemitones(3, 0)
+    outs = []
+    o.seek(x[:, :3000], 1.0)
+    outs.append(o.process(x[:, 3000:7800], 4800))
+    z = np.zeros((1, 30000), np.float32)
+    outs += [o.process(z[:, :12000], 12000), o.process(z[:, :4000], 4000), o.process(z[:, :4000], 5000)]
+    outs.append(o.process(x[:, 8000:17600], 9000))
+    outs.append(o.flush(1000, 1.0))
+    outs.append(o.process(x[:, 20000:24800], 4800))
+    outs.append(o.flush(5000, 1.1))
+    o.reset()
+    outs.append(o.process(x[:, 20000:24800], 2400))
+    o.outputSeek(x[:, : o.outputSeekLength(1.3)])
+    outs.append(o.process(x[:, 5000:11240], 4800))
+    outs.append(o.exact(x[:, :40000], 50000)[1])
+    return np.concatenate(outs, axis=1)

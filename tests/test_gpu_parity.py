@@ -480,13 +480,12 @@ def test_benchmark_shape_vs_oracle(gpu, oracle_port, name, S, calls):
     assert whole.max() <= 1e-2, (whole.max(), np.median(whole))
     lvl = np.array([20 * np.log10(rms(y[s]) / rms(ref[i])) for i, s in enumerate(sampled)])
     assert np.abs(lvl).max() <= 0.1, lvl
-    from oracle import wasmref
-
-    if wasmref.available() and name == "config2_stereo_0p8x":
-        w = wasmref.WasmStretch()
-        cfg(w)
-        rw = signals.run_single(w, x[sampled[0]], ratio, n_out)
-        ref_vs_ref = rms(rw - ref[0])
+    if name == "config2_stereo_0p8x":
+        # the shipped binary's output for this stream, at evenly spaced positions (tests/golden/make_golden.py)
+        g = np.load(os.path.join(GOLD, "config2_bench_shape_wasm.npz"))
+        assert np.array_equal(signals.digest(x[sampled[0]]), g["x_sha256"])
+        idx = signals.sample_positions(ref[0].shape[-1], g["wasm"].shape[-1])
+        ref_vs_ref = rms(g["wasm"] - ref[0][:, idx])
         print("reference (shipped binary) vs oracle over %d blocks: %.2e RMS; GPU vs oracle: %.2e" % (32 * calls, ref_vs_ref, whole[0]))
         assert ref_vs_ref >= 1e-3, ref_vs_ref  # (3.96e-3 measured: the reference does not meet 1e-3 against itself at this horizon)
     # copies of the same input in different batch lanes agree bit for bit
